@@ -1,9 +1,11 @@
 #!/usr/bin/env python3
 """Headline benchmark: BERT-base masked-LM training throughput (samples/s, whole job).
 
-Contract (see task statement): ``python bench.py --gpus N --steps K --warmup W`` (for N>1 the same
-command under ``torch.distributed.run``); W untimed steps, then exactly K steps timed on the device
-with CUDA events between barrier+synchronize pairs, MAX over ranks, one JSON line from rank 0.
+``python bench.py --gpus N --steps K --warmup W`` (for N>1 the same command under
+``torch.distributed.run``): W untimed steps, then exactly K steps timed on the device with CUDA events
+between barrier+synchronize pairs, MAX over ranks, one JSON line from rank 0.  Weights, batches and
+dropout are seeded, so the same arguments give the same inputs on every run; ``--dump-outputs DIR``
+writes what the last timed step returned (see ``dump_outputs``) to compare two builds output for output.
 
 Metric/config = BASELINE.json config 2 / BASELINE.md B1: ``bert_base`` (12L-768-3072-12H, vocab
 30,522, rel-pos bias), fp16 with dynamic loss scaling, Adam(0.9, 0.98, eps 1e-6), clip-norm 1.0,
@@ -46,6 +48,9 @@ def parse():
                          "gencode into baseline/_ref_ext by baseline/build_ref_ext.sh) = BASELINE.md B2; the default "
                          "reference arm is its stock install without extensions (B1)")
     ap.add_argument("--report-losses", action="store_true", help="add the losses read back in the end-to-end region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's logging output and a seeded sample of the "
+                         "updated weights to DIR/<name>.npy (rank 0)")
     ap.add_argument("--sync-overflow-check", action="store_true",
                     help="ours: read the grad norm on the host every step (reference behaviour) instead of the "
                          "deferred, device-side overflow skip")
@@ -249,12 +254,38 @@ def build_trainer(a, impl, world, rank, local_rank):
     args = options.parse_args_and_arch(parser, input_args=flags)
     args.distributed_rank = rank
     args.device_id = local_rank
+    torch.manual_seed(args.seed)  # the initial weights
     task = tasks.setup_task(args)
     model = task.build_model(args)
     loss = task.build_loss(args)
     trainer = Trainer(args, task, model, loss)
     trainer._total_train_steps = args.max_update  # what init_total_train_steps() would set
     return args, task, trainer
+
+
+DUMP_PARAM_SAMPLE = 1 << 22  # 16 MB of float32
+TIMING_STATS = ("wall", "train_wall", "ups", "gb_free")  # differ from run to run by nature
+
+
+def dump_outputs(out_dir, stats, model):
+    """What a caller of ``Trainer.train_step`` receives from the step: its logging output (one float64 array per
+    numeric statistic, timing meters left out) and the updated model, as ``params_sample.npy``: float32 values at
+    2^22 positions of all parameters flattened in ``named_parameters()`` order, drawn (with replacement) from a fixed
+    seed."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, value in stats.items():
+        if name in TIMING_STATS:
+            continue
+        arr = np.asarray(value.detach().cpu().double().numpy() if torch.is_tensor(value) else value)
+        if arr.dtype.kind in "biuf":
+            np.save(os.path.join(out_dir, name + ".npy"), arr.astype(np.float64))
+    with torch.no_grad():
+        flat = torch.cat([p.detach().reshape(-1).float() for _, p in model.named_parameters()])
+        idx = torch.from_numpy(np.sort(np.random.RandomState(0).randint(0, flat.numel(), size=DUMP_PARAM_SAMPLE)))
+        np.save(os.path.join(out_dir, "params_sample.npy"), flat[idx.to(flat.device)].cpu().numpy())
 
 
 def count_launches_start(impl):
@@ -338,14 +369,13 @@ def main():
     seen_losses = []
 
     def run_steps(batches, n, read_loss):
-        last = None
+        out = None
         for i in range(n):
             out = trainer.train_step(split_micro(batches[i % len(batches)]))
             if read_loss and out is not None:
                 v = out.get("loss", None)
-                last = float(v) if v is not None else None  # device -> host read of the step result
-                seen_losses.append(last)
-        return last
+                seen_losses.append(float(v) if v is not None else None)  # device -> host read of the step result
+        return out
 
     # ---- warm-up (builds optimizer, allocator high-water mark, cuBLAS heuristics, loss scale) ----
     run_steps(on_device, max(3, a.warmup), read_loss=False)
@@ -359,12 +389,16 @@ def main():
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     start.record()
-    run_steps(on_device, a.steps, read_loss=False)
+    last_out = run_steps(on_device, a.steps, read_loss=False)
     stop.record()
     barrier()
     launches = count_launches_stop(a.impl)
     elapsed_ms = start.elapsed_time(stop)
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        if last_out is None:
+            raise RuntimeError("the last timed step returned no logging output (an fp16 overflow skipped it)")
+        dump_outputs(a.dump_outputs, last_out, trainer.get_model())
     t = torch.tensor([elapsed_ms], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
